@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- images/sec for the full adversarial G+D step (BASELINE.json metric) on synthetic 64x64x3 batches.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c4|c5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path (SURVEY.md 8d): x_fake = G(z_d); D update on (x_real, y_real)+(x_fake, y_fake);
@@ -20,6 +20,10 @@ Workload at N=1: BASELINE configs[1] = 64x64x3 DCGAN, z=100, bf16, batch 128 per
             oneDNN/MKL port or the NumPy oracle instead.
 `extra`   : short runs of the other BASELINE configurations (C4 128x128, C5 MLP-GAN) so that the driver's record carries them.
 --impl reference: that CPU restatement IS the reference arm (DL4J itself cannot run: no JVM in the image; SURVEY.md 8c).
+--dump-outputs DIR: after the K timed steps, rank 0 writes what the last of them left to a caller, as float32 .npy files: `losses`
+            (D real, D fake, G) and the flattened parameters `generator_params` / `discriminator_params` (DL4J order, BatchNorm running
+            statistics included).  Inputs and initial parameters are seeded, so two builds run with the same arguments compare element for
+            element.  The files stay under 64 MB: when the parameters are larger (C4), each keeps a fixed seeded sample of its elements.
 """
 from __future__ import annotations
 
@@ -35,6 +39,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only: the benchmark writes nothing into it
+DUMP_BYTES = 63_000_000                 # --dump-outputs: array bytes, leaving room for the .npy headers under 64 MB
 
 CONFIGS = {
     # name: (image size, z, nf, nc, per-GPU batch)
@@ -210,7 +216,7 @@ def cpu_step_rate(cfg_name, batch, steps, warmup, budget_s=None):
 def run_reference(args, cfg, rank, world):
     if rank != 0:
         return
-    steps, warmup = max(1, args.steps), max(1, args.warmup)
+    steps, warmup = args.steps, max(1, args.warmup)
     ips, sec, sample, engine, cores = cpu_step_rate(args.config, cfg["batch"], steps, warmup, budget_s=150.0)     # exactly K timed steps
     unit = "samples/s" if cfg.get("mlp") else "images/s"
     line = {
@@ -340,6 +346,20 @@ def timed_resident_steps(ctx, gan, n, steps, warmup, barrier):
     return step_ms
 
 
+def dump_outputs(path, arrays, budget=DUMP_BYTES):
+    """Writes each array as <path>/<name>.npy, flattened float32.  Arrays above 1 MiB share what the small ones leave of `budget`; when they
+    do not fit, each keeps a seeded sample of its elements (sorted positions that depend only on its size, so runs stay comparable)."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, np.float32).ravel() for k, v in arrays.items()}
+    big = [k for k, v in arrays.items() if v.nbytes > 1 << 20]
+    small = sum(v.nbytes for k, v in arrays.items() if k not in big)
+    frac = min(1.0, (budget - small) / max(1, sum(arrays[k].nbytes for k in big)))
+    for k, v in arrays.items():
+        if k in big and frac < 1.0:
+            v = v[np.sort(np.random.default_rng(0).choice(v.size, int(v.size * frac), replace=False))]
+        np.save(os.path.join(path, k + ".npy"), v)
+
+
 def run_ours(args, cfg, rank, world, local_rank):
     import torch
     import gan_deeplearning4j_b200 as b
@@ -402,6 +422,8 @@ def run_ours(args, cfg, rank, world, local_rank):
     launches = ctx.launch_count() - launches0; simt = G.simt_gemm_calls() + D.simt_gemm_calls() - simt0
     clocks = sampler.stop() if rank == 0 else None
     losses = gan.losses()
+    if args.dump_outputs and rank == 0:        # before the e2e steps and the roofline legs train or perturb the nets further
+        dump_outputs(args.dump_outputs, {"losses": losses, "generator_params": G.params(), "discriminator_params": D.params()})
     total_ms = float(sum(step_ms))
     # ---- end to end through the host-buffer entry point
     lo = np.zeros(3, np.float32)
@@ -475,7 +497,13 @@ def main():
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS))
     ap.add_argument("--no-cpu", dest="no_cpu", action="store_true", help="skip the cpu_baseline leg (A/B runs of kernel switches; not for reported lines)")
     ap.add_argument("--no-extra", dest="no_extra", action="store_true", help="skip the short C4 / C5 runs appended under `extra`")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="write the losses and parameters left by the last timed step as DIR/<name>.npy (float32, under 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: use it with --impl ours")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     cfg = CONFIGS[args.config]
     if args.impl == "reference":

@@ -84,6 +84,23 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert line["value"] > 0
 
 
+def test_bench_dump_outputs_stay_under_budget_and_repeat(tmp_path):
+    """bench.py --dump-outputs: small arrays are written whole, large ones share the byte budget as seeded samples that repeat run to run."""
+    import bench
+    arrays = {"losses": np.array([0.5, -1.0, 2.0]), "a": np.arange(400_000, dtype=np.float64), "b": -np.arange(300_000)}
+    for d in ("x", "y"):
+        bench.dump_outputs(str(tmp_path / d), arrays, budget=1_000_000)
+    got = {k: np.load(tmp_path / "x" / f"{k}.npy") for k in arrays}
+    assert all(v.dtype == np.float32 and v.ndim == 1 for v in got.values())
+    assert np.array_equal(got["losses"], arrays["losses"])
+    assert sum(v.nbytes for v in got.values()) <= 1_000_000 and got["a"].size > got["b"].size > 0
+    assert np.all(np.diff(got["a"]) > 0) and np.isin(got["a"], arrays["a"]).all()           # sorted sample of the original elements
+    for k in arrays:
+        assert np.array_equal(got[k], np.load(tmp_path / "y" / f"{k}.npy")), k
+    bench.dump_outputs(str(tmp_path / "z"), {"a": arrays["a"]}, budget=10_000_000)
+    assert np.array_equal(np.load(tmp_path / "z" / "a.npy"), arrays["a"])                   # under the budget: written whole
+
+
 def test_checkpoint_container_round_trip_and_nd4j_stream_layout(tmp_path):
     """ModelSerializer-style zip (J:606-618): round trip, and the byte layout of the ND4J stream restated in serializer.py."""
     import io
